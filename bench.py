@@ -1,6 +1,7 @@
 """Benchmark of the DBNet -> PARSeq OCR hot path (BASELINE.json metric) on N B200s of one node.
 
     python bench.py --gpus 1 --steps K --warmup W               # this repo's CUDA path
+    python bench.py ... --dump-outputs DIR                      # + the last timed step's outputs as DIR/*.npy
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...                        # the reference's CPU implementation (oracle restatement)
 
@@ -202,6 +203,50 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------ GPU arm helpers
+DUMP_PROB_VALUES = 1 << 22      # probability-map values kept by --dump-outputs (16 MB of ~120 MB per step)
+
+
+def dump_outputs(out_dir, prefix, prob_dev, post, rec_out):
+    """--dump-outputs: what the last timed step handed its caller, as out_dir/<prefix><name>.npy (float32 / float64,
+    ~20 MB with the default --pages), so that two builds can be compared output for output on identical inputs:
+      det_prob_sample        the detector's probability maps (pages, H, W), values at DUMP_PROB_VALUES fixed positions
+                             (ascending flat indices drawn with numpy seed 0)
+      post_meta              (pages, 4) of the device post-processing front: runs, components, 4 x Euler number, overflow
+      post_runs              (n, 6) = page, root, y, x0, x1, sum of every row run of the last detector batch's pages,
+                             sorted by (page, y, x0)
+      rec_ids, rec_probs     (crops, S) token ids / probabilities of every crop, mini-batch groups in bench order
+      rec_group_steps        (groups,) decode steps of every mini-batch group
+    `post` = (meta, runs, first page of the last detector batch) or None when the front did not run."""
+    from yomitoku_b200.models import DB_RUN_DTYPE
+    os.makedirs(out_dir, exist_ok=True)
+    flat = prob_dev.reshape(-1)
+    n = flat.numel()
+    if n > DUMP_PROB_VALUES:
+        idx = np.sort(np.random.default_rng(0).choice(n, DUMP_PROB_VALUES, replace=False))
+        flat = flat[torch.from_numpy(idx).to(flat.device)]
+    arrays = {"det_prob_sample": flat.cpu().numpy().astype(np.float32)}
+    if post is not None:
+        meta, runs, first = post
+        meta = meta.cpu().numpy()
+        runs = runs.cpu().numpy()
+        rows = []
+        for j in range(meta.shape[0] - first):
+            r = runs[j].reshape(-1).view(DB_RUN_DTYPE)[:min(int(meta[first + j, 0]), runs.shape[1])]
+            rows.append(np.stack([np.full(len(r), first + j, np.float64)] +
+                                 [r[f].astype(np.float64) for f in ("root", "y", "x0", "x1", "sum")], axis=1))
+        rows = np.concatenate(rows)
+        arrays["post_meta"] = meta.astype(np.float64)
+        arrays["post_runs"] = rows[np.lexsort((rows[:, 3], rows[:, 2], rows[:, 0]))]
+    arrays["rec_ids"] = np.concatenate([ids for ids, _, _ in rec_out]).astype(np.float32)
+    arrays["rec_probs"] = np.concatenate([probs for _, probs, _ in rec_out]).astype(np.float32)
+    arrays["rec_group_steps"] = np.array([glen for _, _, glen in rec_out], np.float32)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), a)
+    print("[bench] outputs of the last timed step: %s (%.1f MB)" % (
+        ", ".join("%s%s %s" % (prefix, k, tuple(a.shape)) for k, a in arrays.items()),
+        sum(a.nbytes for a in arrays.values()) / 2**20), file=sys.stderr, flush=True)
+
+
 def _gemm_window(L, fn):
     from yomitoku_b200 import _lib
     f, ms, n = ctypes.c_double(0), ctypes.c_double(0), ctypes.c_longlong(0)
@@ -336,7 +381,11 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip other_configs (config 2, config 3, EOS run)")
     ap.add_argument("--no-window", action="store_true", help="skip the instrumented per-launch GEMM timing step "
                                                                "(for runs under ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -454,7 +503,7 @@ def main():
             ev[0].record()
             det_step()
             ev[1].record()
-            rec_step()
+            rec_out = rec_step()
             ev[2].record()
             torch.cuda.synchronize()
             det_ms += ev[0].elapsed_time(ev[1])
@@ -467,6 +516,9 @@ def main():
     ar_steps = int(L.ytk_parseq_last_steps(rec.model._ensure()))
     phase_value = rec.model.last_phase_ms()     # CUDA-event phase times of the last recognizer call of the timed region
     rec_flops_local = rec.model.last_flops()
+    if args.dump_outputs:
+        post = (post_meta, post_runs, (P - 1) // ocr.det_batch * ocr.det_batch) if det.device_post else None
+        dump_outputs(args.dump_outputs, "rank%d_" % rank if world > 1 else "", prob_dev, post, rec_out)
     tm = torch.tensor([total_ms, det_ms, rec_ms], dtype=torch.float64, device="cuda")
     cnt = torch.tensor([float(n_crops), float(x_value["exchange_bytes_sent"]), float(x_value["exchange_ms"]),
                         rec_flops_local], dtype=torch.float64, device="cuda")

@@ -269,7 +269,8 @@ def test_batched_pipeline_with_stub_models():
         return ids, np.full((n, S), 0.5, np.float32), np.full((n_groups,), S, np.int32)
 
     rec.model.run_packed_ptr = fake_ptr
-    ocr = BatchedOCR(det, rec, workers=2, det_batch=1)
+    # the host crop path (the default only where no GPU is present): the stand-in reads the crop arena on the host
+    ocr = BatchedOCR(det, rec, workers=2, det_batch=1, device_crops=False)
     try:
         got = list(ocr.stream(batches, lookahead=2, prob_override=maps))
         again = [ocr(pg, prob_override=pm) for pg, pm in zip(batches, maps)]
@@ -315,6 +316,7 @@ def test_batched_pipeline_device_crops_with_stub_models(monkeypatch):
 
     host = ctypes.CDLL(build_crop_host.build())
     det = TextDetector(from_pretrained=False, device="cpu")
+    det.device_post = False         # the maps stay host arrays: the post-processing runs on the host, GPU or not
     rec = TextRecognizer(model_name="parseq-tiny-dynw-v4", from_pretrained=False, device="cpu", dynamic_width=True,
                          batch_bucketing=True)
     Hn, Wn = 1184, 1600

@@ -1,13 +1,13 @@
 """CPU: the recognizer's whole HOST flow (rows R4, R5, R10, R11 + orientation fallback + source_downscale) of the
 product against the REFERENCE's own `TextRecognizer.__call__`.
 
-The reference class is executed from /root/reference (oracle/refcheck.py: build_reference_recognizer_shell; its
+The reference class is executed from the reference tree (oracle/refcheck.py: build_reference_recognizer_shell; its
 uninstallable imports are stubs, ParseqDataset / data functions / tokenizer are the real files) with a stand-in PARSeq
 whose output is a function of (crop pixels, padded width, mini-batch length); the product runs the same stand-in behind
 its two device entry points (tests/flow_standins.py).  Equal contents / scores / directions / points therefore mean:
 same crops, same bucketing order, same mini-batches and padding, same result pairing and order restoration, same
-fallback decisions.  tests/golden/flow_ref.npz stores the reference's outputs so the check also runs where
-/root/reference is absent; with the reference present it is also run live."""
+fallback decisions.  tests/golden/flow_ref.npz and tests/golden/live_ref.npz store the reference's outputs, so the
+tests need no reference tree."""
 import ctypes
 import os
 import sys
@@ -19,7 +19,7 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
 import flow_standins as FS  # noqa: E402
-from oracle import build_crop_host, refcheck  # noqa: E402
+from oracle import build_crop_host  # noqa: E402
 
 
 @pytest.fixture()
@@ -85,15 +85,16 @@ def test_product_flow_matches_reference_fixture(name, device_crops_on_host):
     assert host_res.points == dev_res.points
 
 
-@pytest.mark.skipif(not refcheck.available(), reason="needs /root/reference")
 @pytest.mark.parametrize("name", ["dynw_bucketing", "dropped_quad", "fallback_and_downscale"])
 def test_product_flow_matches_reference_live(name):
-    ref, page, quads = FS.reference_recognizer(name)
-    rec, _, _ = FS.product_recognizer(name)
-    r, _ = ref(page, quads)
+    """The product's host-crop path against the reference's contents / scores / directions AND points (stored by
+    tests/golden/make_golden_live.py)."""
+    z = np.load(os.path.join(HERE, "golden", "live_ref.npz"))
+    rec, page, quads = FS.product_recognizer(name)
     p, _ = rec(page, quads)
-    _same(p, r["contents"], r["scores"], r["directions"])
-    assert p.points == r["points"]
+    _same(p, z["flow_%s_contents" % name].tolist(), z["flow_%s_scores" % name],
+          z["flow_%s_directions" % name].tolist())
+    assert p.points == z["flow_%s_points" % name].tolist()
 
 
 def test_detector_flow_matches_reference_fixture():
@@ -108,12 +109,19 @@ def test_detector_flow_matches_reference_fixture():
         assert res.scores == z["scores%d" % i].tolist()
 
 
-@pytest.mark.skipif(not refcheck.available(), reason="needs /root/reference")
 def test_detector_flow_matches_reference_live():
-    ref = refcheck.build_reference_detector_shell()
+    """TextDetector.preprocess (shape, sums, a seeded sample of the tensor: bit-equal) and __call__ against the
+    reference's own TextDetector with the stand-in model (stored by tests/golden/make_golden_live.py)."""
+    sys.path.insert(0, os.path.join(HERE, "golden"))
+    from make_golden_live import PRE_SAMPLE, sample_index
+    z = np.load(os.path.join(HERE, "golden", "live_ref.npz"))
     det = FS.product_detector()
-    for page in FS.detector_pages():
-        assert torch.equal(ref.preprocess(page), det.preprocess(page))
-        r, _ = ref(page)
+    for i, page in enumerate(FS.detector_pages()):
+        x = det.preprocess(page)
+        assert tuple(x.shape) == tuple(z["detflow%d_pre_shape" % i])
+        got = x.reshape(-1)[torch.from_numpy(sample_index(x.numel(), PRE_SAMPLE, 200 + i))].numpy()
+        assert np.array_equal(got, z["detflow%d_pre_sample" % i])
+        assert np.allclose([float(x.double().sum()), float((x.double() ** 2).sum())], z["detflow%d_pre_sum" % i],
+                           rtol=1e-10, atol=0)
         p, _ = det(page)
-        assert p.points == r["points"] and p.scores == r["scores"]
+        assert p.points == z["detflow%d_points" % i].tolist() and p.scores == z["detflow%d_scores" % i].tolist()

@@ -1,5 +1,5 @@
 """CPU: the RT-DETRv2 oracle against outputs of the reference's own model files (tests/golden/rtdetr_ref.npz, generated
-by tests/golden/make_golden_rtdetr.py; live against /root/reference where it exists), and the product's host code
+by tests/golden/make_golden_rtdetr.py; a batch of 2 in tests/golden/live_ref.npz), and the product's host code
 around the device model - LayoutParser / TableStructureRecognizer pre- and post-processing, RTDETRPostProcessor -
 against outputs of the reference's own layout_parser.py / table_structure_recognizer.py
 (tests/golden/rtdetr_wrappers_ref.json)."""
@@ -11,7 +11,6 @@ import numpy as np
 import pytest
 import torch
 
-from oracle import refcheck as rc
 from oracle import rtdetr as R
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -29,8 +28,14 @@ def test_oracle_reproduces_reference_outputs(kind):
     sd = R.make_state_dict(spec, seed=CASES[kind][0])
     aux = {}
     out = R.forward(sd, spec, rtdetr_input(CASES[kind][1]), aux)
-    assert np.abs(out["pred_logits"][0].numpy() - GOLD[kind + "_logits"]).max() < 5e-4
-    assert np.abs(out["pred_boxes"][0].numpy() - GOLD[kind + "_boxes"]).max() < 2e-5
+    # queries come in descending encoder score: on another CPU two (nearly) tied anchors may swap places, so the rows
+    # are compared as a set (ordered by their box), as in the batch-2 test below
+    def rows(boxes, logits):
+        m = np.concatenate([boxes, logits], axis=1)
+        return m[np.lexsort(np.round(m[:, :4], 4).T[::-1])]
+    d = np.abs(rows(out["pred_boxes"][0].numpy(), out["pred_logits"][0].numpy()) -
+               rows(GOLD[kind + "_boxes"], GOLD[kind + "_logits"]))
+    assert d[:, :4].max() < 2e-5 and d[:, 4:].max() < 5e-4
     for i in range(3):
         for name, t in (("c", aux["backbone"][i]), ("e", aux["encoder"][i])):
             ref = GOLD["%s_%s%d" % (kind, name, i + 3)]
@@ -43,13 +48,14 @@ def test_oracle_reproduces_reference_outputs(kind):
     assert all(abs(GOLD[kind + "_enc_scores"][a] - cut) < 1e-3 for a in ref_set ^ got)
 
 
-@pytest.mark.skipif(not rc.available(), reason="needs /root/reference")
 def test_oracle_against_live_reference_batch2():
+    """Batch 2 of the table configuration against the reference's RTDETRv2 outputs stored by
+    tests/golden/make_golden_live.py."""
     spec = R.SPECS["table"]
     sd = R.make_state_dict(spec, seed=5)
     x = rtdetr_input(6, n=2)
-    with torch.no_grad():
-        ref = rc.build_reference_rtdetr(spec.num_classes, sd)(x)
+    z = np.load(os.path.join(HERE, "golden", "live_ref.npz"))
+    ref = {"pred_boxes": torch.from_numpy(z["rtdetr_b2_boxes"]), "pred_logits": torch.from_numpy(z["rtdetr_b2_logits"])}
     out = R.forward(sd, spec, x)
     for b in range(2):
         # queries come in descending encoder score: two anchors with (nearly) the same score may swap places, so the
