@@ -74,6 +74,13 @@ int ytk_op_attention_f16(const void* Q, long long ldq, long long q_rows, const v
                          long long kv_rows, void* O, long long ldo, const ytk_attn_seq* seqs_dev, int nseq, int max_q_len,
                          int heads, int head_dim, int masked, int impl, void* cuda_stream);
 
+/* RT-DETRv2 query selection: per image, the indices of the K largest of L fp32 scores in descending order, equal scores
+ * by ascending index (torch.topk(scores, K) of reference models/layers/rtdetrv2_decoder.py:730).  scores_dev
+ * [n_img, L] and out_idx_dev [n_img, K] int32 are device memory.  L <= 16384: one bitonic sort in shared memory; up to
+ * L = 45056 with K <= 2048: radix select + sort of the K selected (the 960 x 960 cell detector has L = 18900, K = 1500).
+ * Other sizes return an error. */
+int ytk_op_rt_topk_f32(const float* scores_dev, int n_img, int L, int K, int* out_idx_dev, void* stream);
+
 /* ---- Device-side front half of the DBNet post-processing (reference postprocessor/dbnet_postporcessor.py:39-82:
  * binarize, findContours, and the pixel work of minAreaRect / box_score_fast).  One record per horizontal run of an
  * 8-connected component of (prob > thresh). ---- */
@@ -239,6 +246,8 @@ int ytk_rtdetr_device(const ytk_rtdetr* h);
 int ytk_rtdetr_forward_f32(ytk_rtdetr* h, const float* x, int x_on_device, int n, float* pred_logits, float* pred_boxes,
                            int out_on_device, void* cuda_stream);
 double ytk_rtdetr_flops(ytk_rtdetr* h, int n);
+/* device bytes of the activation buffers of the batch-n launch plan (built on first use, like a forward), -1 on error */
+long long ytk_rtdetr_device_bytes(ytk_rtdetr* h, int n);
 /* test hook: copies an intermediate activation (by name, see rtdetr_engine.cu) of the LAST forward of batch size n to
  * the host as fp32; shape4 = {n, h, w, c} (token matrices: {1, 1, rows, c}) */
 int ytk_rtdetr_debug_tensor(ytk_rtdetr* h, int n, const char* name, float* host_out, long long capacity, int* shape4);

@@ -38,6 +38,8 @@ def _declare(lib):
     lib.ytk_op_attention_f16.restype = c_int
     lib.ytk_op_attention_f16.argtypes = [c_void_p, c_ll, c_ll, c_void_p, c_void_p, c_ll, c_ll, c_void_p, c_ll, c_void_p,
                                          c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]
+    lib.ytk_op_rt_topk_f32.restype = c_int
+    lib.ytk_op_rt_topk_f32.argtypes = [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]
 
 
 class YtkAttnSeq(ctypes.Structure):
@@ -132,6 +134,8 @@ def _declare_rtdetr(lib):
     lib.ytk_rtdetr_forward_f32.argtypes = [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p]
     lib.ytk_rtdetr_flops.restype = ctypes.c_double
     lib.ytk_rtdetr_flops.argtypes = [c_void_p, c_int]
+    lib.ytk_rtdetr_device_bytes.restype = c_ll
+    lib.ytk_rtdetr_device_bytes.argtypes = [c_void_p, c_int]
     lib.ytk_rtdetr_debug_tensor.restype = c_int
     lib.ytk_rtdetr_debug_tensor.argtypes = [c_void_p, c_int, ctypes.c_char_p, c_void_p, c_ll, P(c_int)]
 

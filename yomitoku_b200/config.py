@@ -122,13 +122,14 @@ TextRecognizerPARSeqTinyDynwV4Config = _parseq(_R + "parseq-tiny-dynw-v4", "char
 
 
 # ------------------------------------------------------------------------------------------------ layout models
-def _rtdetr(repo, num_classes, thresh_score, category, role=None):
-    """Values of reference configs/cfg_layout_parser_rtdtrv2{,_v2}.py and cfg_table_structure_recognizer_rtdtrv2.py."""
+def _rtdetr(repo, num_classes, thresh_score, category, role=None, img=640, num_queries=300):
+    """Values of reference configs/cfg_layout_parser_rtdtrv2{,_v2}.py, cfg_table_structure_recognizer_rtdtrv2.py and
+    cfg_table_cell_parser_rtdtrv2.py."""
     def make():
         cfg = {
             "hf_hub_repo": repo,
             "thresh_score": thresh_score,
-            "data": {"img_size": [640, 640]},
+            "data": {"img_size": [img, img]},
             "PResNet": {"depth": 50, "variant": "d", "freeze_at": 0, "return_idx": [1, 2, 3], "num_stages": 4,
                         "freeze_norm": True},
             "HybridEncoder": {"in_channels": [512, 1024, 2048], "feat_strides": [8, 16, 32], "hidden_dim": 256,
@@ -136,8 +137,8 @@ def _rtdetr(repo, num_classes, thresh_score, category, role=None):
                               "dropout": 0.0, "enc_act": "gelu", "expansion": 1.0, "depth_mult": 1, "act": "silu"},
             "RTDETRTransformerv2": {"num_classes": num_classes, "feat_channels": [256, 256, 256],
                                     "feat_strides": [8, 16, 32], "hidden_dim": 256, "num_levels": 3, "num_layers": 6,
-                                    "num_queries": 300, "num_denoising": 100, "label_noise_ratio": 0.5,
-                                    "box_noise_scale": 1.0, "eval_spatial_size": [640, 640], "eval_idx": -1,
+                                    "num_queries": num_queries, "num_denoising": 100, "label_noise_ratio": 0.5,
+                                    "box_noise_scale": 1.0, "eval_spatial_size": [img, img], "eval_idx": -1,
                                     "num_points": [4, 4, 4], "cross_attn_method": "default",
                                     "query_select_method": "default"},
             "category": list(category),
@@ -156,3 +157,8 @@ LayoutParserRTDETRv2V2Config = _rtdetr("KotaroKinoshita/yomitoku-layout-parser-r
                                        _LAYOUT_ROLE)
 TableStructureRecognizerRTDETRv2Config = _rtdetr(
     "KotaroKinoshita/yomitoku-table-structure-recognizer-rtdtrv2-open-beta", 3, 0.4, ["row", "col", "span"])
+# the cell detector was trained with 900 queries; it runs 1500 at inference (the weights do not depend on the count) so
+# that dense tables of up to ~1000 cells stay below the detection limit
+TableCellParserRTDETRv2Config = _rtdetr("KotaroKinoshita/yomitoku-cell-detector-rtdtrv2-v1", 6, 0.5,
+                                        ["table", "cell", "header", "empty", "kv_item", "grid"], img=960,
+                                        num_queries=1500)

@@ -173,6 +173,14 @@ int ytk_op_attention_f16(const void* Q, long long ldq, long long q_rows, const v
                : YTK_OK;
 }
 
+int ytk_op_rt_topk_f32(const float* scores_dev, int n_img, int L, int K, int* out_idx_dev, void* stream) {
+    if (!scores_dev || !out_idx_dev || n_img < 1 || L < 1 || K < 1) {
+        ytk::set_error("ytk_op_rt_topk_f32: bad arguments (n_img %d, L %d, K %d)", n_img, L, K);
+        return YTK_ERR;
+    }
+    return ytk::launch_rt_topk(scores_dev, n_img, L, K, out_idx_dev, static_cast<cudaStream_t>(stream)) ? YTK_ERR : YTK_OK;
+}
+
 static_assert(sizeof(ytk_db_run) == sizeof(ytk::DbRun), "ytk_db_run and ytk::DbRun must have one layout");
 
 int ytk_dbnet_post_front(const float* prob_dev, int n_pages, int H, int W, float thresh, void* scratch_dev,
@@ -631,6 +639,13 @@ double ytk_rtdetr_flops(ytk_rtdetr* h, int n) {
     DevGuard dev_guard(h->device);
     ytk::RtdetrEngine* e = rt_engine(h, n);
     return e ? e->flops : -1.0;
+}
+
+long long ytk_rtdetr_device_bytes(ytk_rtdetr* h, int n) {
+    std::lock_guard<std::mutex> lk(h->mu);
+    DevGuard dev_guard(h->device);
+    ytk::RtdetrEngine* e = rt_engine(h, n);
+    return e ? (long long)e->total_bytes : -1;
 }
 
 int ytk_rtdetr_debug_tensor(ytk_rtdetr* h, int n, const char* name, float* host_out, long long capacity, int* shape4) {

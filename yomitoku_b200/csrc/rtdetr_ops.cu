@@ -153,6 +153,119 @@ __global__ void topk_kernel(const float* __restrict__ scores, int L, int NP, int
         out_idx[(long long)blockIdx.x * K + i] = 0x7fffffff - (int)(keys[i] & 0xffffffffu);
 }
 
+// The same result as topk_kernel for anchor counts whose full sort does not fit shared memory (the 960 cell detector:
+// 18900 anchors).  One CTA of 1024 threads per image.  The scores stay in shared memory as 32-bit monotone keys; an
+// MSB-first radix select (8 bits per pass) over the 48-bit key v = (score key << 16) | (0xffff - anchor) - the composite
+// topk_key restricted to the bits that differ when L <= 65536 - finds the smallest prefix t such that exactly K keys have
+// v >= t.  Those K keys are compacted into a next_pow2(K) buffer and bitonic-sorted (descending).  Every v is distinct,
+// so the selected set and the order are fully determined; the passes over the anchor bits only run while scores tie.
+constexpr int kSelThreads = 1024;
+__device__ __forceinline__ unsigned score_key(float s) {
+    const unsigned u = __float_as_uint(s);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);          // the map of topk_key
+}
+__global__ void __launch_bounds__(kSelThreads, 1)
+topk_select_kernel(const float* __restrict__ scores, int L, int NK, int K, int* __restrict__ out_idx) {
+    extern __shared__ unsigned long long sel_smem[];
+    unsigned long long* sel = sel_smem;                                     // [NK] selected composite keys
+    unsigned* hist = reinterpret_cast<unsigned*>(sel_smem + NK);            // [256]
+    unsigned* skey = hist + 256;                                            // [L] score keys
+    __shared__ unsigned long long s_prefix;    // digits chosen so far
+    __shared__ unsigned s_need, s_cnt, s_n;    // keys still to take inside the prefix bucket, size of the chosen bucket
+    const int tid = threadIdx.x, lane = tid & 31;
+    const float* s = scores + (long long)blockIdx.x * L;
+    for (int i = tid; i < L; i += kSelThreads) skey[i] = score_key(s[i]);
+    if (tid == 0) {
+        s_prefix = 0;
+        s_need = K;
+        s_n = 0;
+    }
+    int shift = 40;
+    for (;; shift -= 8) {
+        for (int i = tid; i < 256; i += kSelThreads) hist[i] = 0;
+        __syncthreads();
+        const unsigned long long prefix = s_prefix;
+        for (int base = 0; base < L; base += kSelThreads) {
+            const int i = base + tid;
+            unsigned long long v = 0;
+            bool in = false;
+            if (i < L) {
+                v = ((unsigned long long)skey[i] << 16) | (unsigned)(0xffff - i);
+                in = (v >> (shift + 8)) == prefix;
+            }
+            const unsigned m = __ballot_sync(0xffffffffu, in);
+            if (in) {
+                // lanes with the same digit add once: quantised or blank-crop scores put thousands of keys in one bucket
+                const unsigned d = (unsigned)(v >> shift) & 0xffu;
+                const unsigned peers = __match_any_sync(m, d);
+                if (lane == __ffs(peers) - 1) atomicAdd(&hist[d], __popc(peers));
+            }
+        }
+        __syncthreads();
+        if (tid < 32) {
+            // lane l holds the bins 255 - 8 l down to 248 - 8 l; a scan over the lanes counts the keys in higher bins
+            const unsigned need = s_need;
+            unsigned c[8], sum = 0;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+                c[j] = hist[255 - 8 * lane - j];
+                sum += c[j];
+            }
+            unsigned incl = sum;
+#pragma unroll
+            for (int off = 1; off < 32; off <<= 1) {
+                const unsigned t = __shfl_up_sync(0xffffffffu, incl, off);
+                if (lane >= off) incl += t;
+            }
+            unsigned above = incl - sum;
+            if (above < need && need <= incl) {            // the bucket of the need-th largest key is in this lane
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                    if (above + c[j] >= need) {
+                        s_prefix = (prefix << 8) | (unsigned)(255 - 8 * lane - j);
+                        s_need = need - above;
+                        s_cnt = c[j];
+                        break;
+                    }
+                    above += c[j];
+                }
+            }
+        }
+        __syncthreads();
+        if (s_cnt == s_need) break;                        // the prefix buckets hold exactly K keys (at the latest at shift 0)
+    }
+    const unsigned long long thr = s_prefix << shift;
+    for (int base = 0; base < L; base += kSelThreads) {
+        const int i = base + tid;
+        bool take = false;
+        if (i < L) take = (((unsigned long long)skey[i] << 16) | (unsigned)(0xffff - i)) >= thr;
+        const unsigned m = __ballot_sync(0xffffffffu, take);
+        unsigned pos = 0;
+        if (lane == 0 && m) pos = atomicAdd(&s_n, __popc(m));
+        pos = __shfl_sync(0xffffffffu, pos, 0);
+        if (take) sel[pos + __popc(m & ((1u << lane) - 1))] = ((unsigned long long)skey[i] << 32) | (unsigned)(0x7fffffff - i);
+    }
+    for (int i = K + tid; i < NK; i += kSelThreads) sel[i] = 0ull;        // below every real key
+    __syncthreads();
+    for (int k = 2; k <= NK; k <<= 1)
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            for (int i = tid; i < NK; i += kSelThreads) {
+                const int p = i ^ j;
+                if (p > i) {
+                    const unsigned long long a = sel[i], b = sel[p];
+                    const bool desc = (i & k) == 0;
+                    if (desc ? (a < b) : (a > b)) {
+                        sel[i] = b;
+                        sel[p] = a;
+                    }
+                }
+            }
+            __syncthreads();
+        }
+    for (int i = tid; i < K; i += kSelThreads)
+        out_idx[(long long)blockIdx.x * K + i] = 0x7fffffff - (int)(sel[i] & 0xffffffffu);
+}
+
 // decoder start: target rows = output_memory[top-k rows] (fp32 + fp16), anchors of the selected positions
 __global__ void gather_queries_kernel(const float* __restrict__ om, int D, const int* __restrict__ idx, int K, RtLevels lv,
                                       int n_img, float* __restrict__ tgt, op_t* __restrict__ tgt16,
@@ -328,18 +441,41 @@ int launch_rt_topk(const float* scores, int n_img, int L, int K, int* out_idx, c
     int NP = 1;
     while (NP < L) NP <<= 1;
     const size_t smem = (size_t)NP * sizeof(unsigned long long);
+    if (smem > (size_t)kTopkSmemBytes) return launch_rt_topk_select(scores, n_img, L, K, out_idx, st);
     static unsigned long long attr_done = 0;   // per device
     if (first_launch_on_device(&attr_done)) {
-        if (cudaFuncSetAttribute(topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess) {
+        if (cudaFuncSetAttribute(topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTopkSmemBytes) != cudaSuccess) {
             set_error("topk: cannot raise the shared memory limit");
             return 1;
         }
     }
-    if (smem > 200 * 1024 || K > L) {
+    if (K > L) {
         set_error("topk: %d candidates / k = %d unsupported", L, K);
         return 1;
     }
     topk_kernel<<<n_img, 1024, smem, st>>>(scores, L, NP, K, out_idx);
+    count_launch();
+    return cudaGetLastError() != cudaSuccess;
+}
+
+int launch_rt_topk_select(const float* scores, int n_img, int L, int K, int* out_idx, cudaStream_t st) {
+    if (L < 1 || L > kTopkSelectMaxL || K < 1 || K > kTopkSelectMaxK || K > L) {
+        set_error("topk: %d candidates / k = %d unsupported (radix select: 1 <= k <= min(%d, candidates), candidates <= %d)",
+                  L, K, kTopkSelectMaxK, kTopkSelectMaxL);
+        return 1;
+    }
+    int NK = 1;
+    while (NK < K) NK <<= 1;
+    const size_t smem = (size_t)NK * sizeof(unsigned long long) + 256 * sizeof(unsigned) + (size_t)L * sizeof(unsigned);
+    static unsigned long long attr_done = 0;   // per device
+    if (first_launch_on_device(&attr_done)) {
+        if (cudaFuncSetAttribute(topk_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTopkSmemBytes) !=
+            cudaSuccess) {
+            set_error("topk: cannot raise the shared memory limit");
+            return 1;
+        }
+    }
+    topk_select_kernel<<<n_img, kSelThreads, smem, st>>>(scores, L, NK, K, out_idx);
     count_launch();
     return cudaGetLastError() != cudaSuccess;
 }

@@ -47,8 +47,19 @@ int launch_rt_mask_invalid(float* x, int D, const float* bias, const int* invali
                            int n_img, cudaStream_t st);
 int launch_rt_enc_scores(const float* logits, long long ldl, int C, const RtLevels& lv, int n_img, float* scores,
                          cudaStream_t st);
-// per image: indices of the K largest of L scores, descending (ties: smaller index first)
+// per image: indices of the K largest of L scores, descending (ties: smaller index first).  A bitonic sort of all L keys
+// in shared memory when next_pow2(L) 8-byte keys fit kTopkSmemBytes (L <= 16384: the 640 models), otherwise
+// launch_rt_topk_select.
+constexpr int kTopkSmemBytes = 200 * 1024;
 int launch_rt_topk(const float* scores, int n_img, int L, int K, int* out_idx, cudaStream_t st);
+// The same result by radix select + a sort of the K selected keys: needs 1 <= K <= min(L, kTopkSelectMaxK) and
+// L <= kTopkSelectMaxL (4 B per score + 8 B per next_pow2(K) key + 1 KB of histogram within kTopkSmemBytes; the kernel's
+// key keeps 16 anchor bits).  Other sizes return an error.
+constexpr int kTopkSelectMaxK = 2048;
+constexpr int kTopkSelectMaxL = 45056;
+static_assert(kTopkSelectMaxL <= 65536, "topk_select_kernel keeps 16 anchor bits");
+static_assert(kTopkSelectMaxL * 4 + kTopkSelectMaxK * 8 + 1024 <= kTopkSmemBytes, "topk_select_kernel shared memory");
+int launch_rt_topk_select(const float* scores, int n_img, int L, int K, int* out_idx, cudaStream_t st);
 int launch_rt_gather_queries(const float* om, int D, const int* idx, int K, const RtLevels& lv, int n_img, float* tgt,
                              void* tgt16, const float* anchors, float* anchor_sel, cudaStream_t st);
 // ref[i] = sigmoid(delta[i] + (anchor_sel ? anchor_sel[i] : inverse_sigmoid(ref[i]))), i over n boxes x 4

@@ -29,11 +29,15 @@ def _area(box):
     return (box[2] - box[0]) * (box[3] - box[1])
 
 
-def filter_contained_rectangles_within_category(category_elements):
+def filter_contained_rectangles_within_category(category_elements, ignore=(), drop_outer=False):
     """Inside every category: a box that lies (> 80 % of its area) inside another one is dropped; of two boxes that
     contain each other the one that is NOT larger is dropped (reference layout_parser.py:31-61; every pair is judged
-    on the original list, a box already dropped still eliminates others)."""
+    on the original list, a box already dropped still eliminates others).  Categories in `ignore` stay as they are.
+    drop_outer: the enclosing box is dropped instead of the enclosed one (the cell detector's rule, reference
+    table_cell_detector.py:41-75; the mutual case is the same)."""
     for category, elements in category_elements.items():
+        if category in ignore:
+            continue
         boxes = [e["box"] for e in elements]
         keep = [True] * len(boxes)
         for i in range(len(boxes)):
@@ -42,9 +46,9 @@ def filter_contained_rectangles_within_category(category_elements):
                 if j_in_i and i_in_j:
                     keep[j if _area(boxes[i]) > _area(boxes[j]) else i] = False
                 elif j_in_i:
-                    keep[j] = False
+                    keep[i if drop_outer else j] = False
                 elif i_in_j:
-                    keep[i] = False
+                    keep[j if drop_outer else i] = False
         category_elements[category] = [e for e, k in zip(elements, keep) if k]
     return category_elements
 

@@ -598,8 +598,9 @@ def _rtdetr_anchors(img=640, strides=(8, 16, 32), grid_size=0.05, eps=1e-2):
     return torch.where(valid, torch.log(a / (1 - a)), torch.inf), valid
 
 
-def _rtdetr_random_state_dict(num_classes, seed=0):
-    """Random init with the reference's key set and shapes (RTDETRv2(cfg).state_dict(), from_pretrained=False)."""
+def _rtdetr_random_state_dict(num_classes, seed=0, img=640):
+    """Random init with the reference's key set and shapes (RTDETRv2(cfg).state_dict(), from_pretrained=False) for an
+    img x img input: the anchor buffers depend on it."""
     g = torch.Generator().manual_seed(seed)
     sd = OrderedDict()
     D, F, L, P, H = 256, 1024, 6, 12, 8
@@ -659,7 +660,7 @@ def _rtdetr_random_state_dict(num_classes, seed=0):
     for i in range(2):
         conv_norm("encoder.lateral_convs.%d" % i, D, D, 1, True)
         conv_norm("encoder.downsample_convs.%d" % i, D, D, 3, True)
-    sd["decoder.anchors"], sd["decoder.valid_mask"] = _rtdetr_anchors()
+    sd["decoder.anchors"], sd["decoder.valid_mask"] = _rtdetr_anchors(img)
     for i in range(3):
         conv_norm("decoder.input_proj.%d" % i, D, D, 1, True)
     prior = -math.log(99.0)
@@ -699,8 +700,9 @@ def _rtdetr_random_state_dict(num_classes, seed=0):
 
 class RTDETRv2(_DeviceModel):
     """reference models/rtdetr.py:9-22 (PResNet-50d + HybridEncoder + RTDETRTransformerv2, eval).  `model(tensor)` takes
-    the (n, 3, 640, 640) fp32 tensor in [0, 1] that LayoutParser / TableStructureRecognizer.preprocess produce and returns
-    {"pred_logits": (n, 300, C), "pred_boxes": (n, 300, 4)} on the tensor's device.  The forward is the sm_100a engine
+    the (n, 3, S, S) fp32 tensor in [0, 1] that LayoutParser / TableStructureRecognizer / CellDetector.preprocess produce
+    (S = cfg.data.img_size: 640, 960 for the cell detector) and returns {"pred_logits": (n, Q, C), "pred_boxes": (n, Q, 4)}
+    (Q = num_queries: 300, 1500 for the cell detector) on the tensor's device.  The forward is the sm_100a engine
     behind ytk_rtdetr_forward_f32 (csrc/rtdetr_engine.cu); there is no CPU fallback."""
 
     def __init__(self, cfg=None, seed=0):
@@ -714,7 +716,7 @@ class RTDETRv2(_DeviceModel):
                                 list(d.eval_spatial_size) != [self.img_size] * 2):
             raise ValueError("RTDETRv2: square img_size == eval_spatial_size expected, got %s / %s"
                              % (list(cfg.data.img_size), list(d.eval_spatial_size)))
-        self._sd = _rtdetr_random_state_dict(self.num_classes, seed)
+        self._sd = _rtdetr_random_state_dict(self.num_classes, seed, self.img_size)
 
     def _ensure(self):
         self._require_cuda()
@@ -757,6 +759,10 @@ class RTDETRv2(_DeviceModel):
 
     def flops(self, n=1):
         return _lib.lib().ytk_rtdetr_flops(self._ensure(), n)
+
+    def device_bytes(self, n=1):
+        """Device bytes of the activation buffers of the batch-n engine."""
+        return int(_lib.lib().ytk_rtdetr_device_bytes(self._ensure(), n))
 
     def debug_tensor(self, n, name):
         """Intermediate activation of the last forward of batch size n (test hook) as a numpy array."""

@@ -1,6 +1,7 @@
 """Result types of the hot path (pydantic), mirroring reference src/yomitoku/schemas/document_analyzer.py:137-180,
-234-254 and BaseSchema (base.py:51-57): extra fields forbidden, assignment validated."""
-from typing import List, Union
+234-254, schemas/table_semantic_parser.py:62-140 (the cell detector's results) and BaseSchema (base.py:51-57): extra
+fields forbidden, assignment validated."""
+from typing import Any, Dict, List, Union
 
 from pydantic import BaseModel, ConfigDict, Field, conlist
 
@@ -117,3 +118,35 @@ class DocumentAnalyzerSchema(BaseSchema):
     tables: List[TableStructureRecognizerSchema] = Field(default_factory=list)
     words: List[WordPrediction] = Field(default_factory=list)
     figures: List[FigureSchema] = Field(default_factory=list)
+
+
+class CellSchema(BaseSchema):
+    """One cell of a cell-detected table (reference schemas/table_semantic_parser.py:62-101).  row / col / spans and
+    contents stay None until a table-semantic parser fills them."""
+    meta: Dict[str, Any] = Field(default_factory=dict, description="Additional metadata for template/semantics")
+    contents: Union[str, None] = Field(..., description="Text content of the cell")
+    role: Union[str, None] = Field(..., description="Role of the cell, e.g., ['cell', 'header', 'empty', 'group']")
+    id: Union[str, None] = Field(..., description="Unique identifier of the cell")
+    box: Box = Field(..., description="Bounding box of the cell in the format [x1, y1, x2, y2]")
+    row: Union[int, None] = Field(..., description="Row index of the cell in the table")
+    col: Union[int, None] = Field(..., description="Column index of the cell in the table")
+    row_span: Union[int, None] = Field(..., description="Number of rows spanned by the cell")
+    col_span: Union[int, None] = Field(..., description="Number of columns spanned by the cell")
+
+
+class RegionSchema(BaseSchema):
+    """A region the cell detector predicts directly (kv_item / grid), reference :104-112."""
+    id: Union[str, None] = Field(None, description="Region id")
+    box: Box = Field(..., description="Bounding box [x1, y1, x2, y2]")
+    role: str = Field(..., description="Region role, e.g., ['kv_item', 'grid']")
+    score: float = Field(1.0, description="Detection score")
+
+
+class TableDetectorSchema(BaseSchema):
+    """What CellDetector returns per table (reference :115-140)."""
+    id: Union[str, None] = Field(..., description="Unique identifier of the table")
+    box: Box = Field(..., description="Bounding box of the table in the format [x1, y1, x2, y2]")
+    role: Union[str, None] = Field(..., description="Role of the table region")
+    cells: List[CellSchema] = Field(..., description="List of detected table cells")
+    kv_regions: List[RegionSchema] = Field(default_factory=list, description="Model-predicted key-value item regions")
+    grid_regions: List[RegionSchema] = Field(default_factory=list, description="Model-predicted grid regions")
